@@ -8,6 +8,10 @@ One "step" = one full time step of the hot path on a uniform grid without bodies
 cell-updates per step = cells * (2 stage sweeps + K Poisson iterations)   [the metric's own definition]
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--level L] [--poisson-iters K] [--impl reference]
+                    [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step handed back (u, v, p and the step's dt, iterations, residual) as .npy
+files, so that two builds run with the same arguments (hence the same seeded inputs) can be compared output for output.
 
 N > 1: launched by torchrun, one rank per GPU; the 8192^2 grid is split into contiguous Hilbert ranges
 (strong scaling); halos and Krylov dots go over NVLink peer memory inside the library's kernels.
@@ -151,7 +155,6 @@ def cpu_composite(level, reps, kiter):
     restatement of cuda.cu for the Poisson iterations (one fixed definition: the figure never switches solver), and the
     composite with the reference's own GPU solver on this box's B200 is reported beside it as `with_reference_gpu_solver`."""
     threads = usable_cpus()
-    reps = max(5, reps)
     run_harness_time(HARNESS, 3, 1, 1, threads, timeout=120)           # warm: binary and OpenMP runtime paged in
     t = run_harness_time(HARNESS, level, reps, kiter, threads, timeout=900)
     val, step_s = _composite(t, kiter)
@@ -238,6 +241,42 @@ def multi_gpu_parity(cup2d_b200, np, torch, dist, rank, world, local_rank, K):
     return out[0]
 
 
+DUMP_CELLS = 1 << 20   # at most this many cells per field in --dump-outputs; larger grids are sampled (u, v, p, index: <= 32 MB)
+
+
+def dump_outputs(path, np, dist, rank, order_loc, nbx, vel, pres, result):
+    """Write u.npy, v.npy, p.npy (float64) at the cells of cell_index.npy (flat index iy*N+ix of the global grid: every cell,
+    or the distinct cells among DUMP_CELLS fixed seeded draws) and step.npy = [dt, iterations, residual] of the last step.
+    vel, pres: this rank's blocks in the reference layout; every rank calls this, rank 0 writes."""
+    N = nbx * 8
+    cells = N * N
+    idx = np.arange(cells) if cells <= DUMP_CELLS else np.unique(np.random.default_rng(0).integers(0, cells, DUMP_CELLS))
+    gy, gx = np.divmod(idx, N)
+    where = np.full((nbx, nbx), -1, dtype=np.int64)   # global block (j, i) -> local block, -1 on other ranks
+    where[order_loc[:, 1], order_loc[:, 0]] = np.arange(len(order_loc))
+    b = where[gy // 8, gx // 8]
+    mine = np.flatnonzero(b >= 0)
+    cell = (b[mine] * 8 + gy[mine] % 8) * 8 + gx[mine] % 8
+    uv = vel.reshape(-1, 2)[cell]
+    parts = [(mine, uv[:, 0], uv[:, 1], pres[cell])]
+    if dist is not None:
+        gathered = [None] * dist.get_world_size()
+        dist.all_gather_object(gathered, parts[0])
+        parts = gathered
+    if rank != 0:
+        return
+    out = {k: np.full(len(idx), np.nan) for k in ("u", "v", "p")}
+    for pos, u, v, p in parts:
+        out["u"][pos], out["v"][pos], out["p"][pos] = u, v, p
+    if cells <= DUMP_CELLS:
+        out = {k: a.reshape(N, N) for k, a in out.items()}
+    out["cell_index"] = idx.astype(np.float64)
+    out["step"] = np.array(result, dtype=np.float64)
+    os.makedirs(path, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 # FP64 instructions the advect stage executes per cell (DFMA + DMUL + DADD of the ncu instruction mix; round 1: 189)
 ADVECT_FP64_PER_CELL = 152.4
 
@@ -256,7 +295,12 @@ def main():
     ap.add_argument("--no-pipeline", action="store_true", help="skip the pipelined end-to-end figure")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel from the host instead of replaying the step graph")
     ap.add_argument("--profile-steps", type=int, default=5, help="steps of the separate, event-instrumented pass (per-kernel table)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the fields and result of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the cup2d_b200 arm only")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -278,7 +322,7 @@ def main():
         if rank != 0:
             return
         try:
-            cb = cpu_composite(args.cpu_level, max(5, args.steps), K)
+            cb = cpu_composite(args.cpu_level, args.steps, K)
         except Exception as ex:  # the reference harness could not be run on this box
             print(json.dumps({"impl": "reference", "unavailable": f"reference harness failed: {type(ex).__name__}: {ex}"[:300]}))
             return
@@ -288,7 +332,7 @@ def main():
                                f"operators, same composite; CPU throughput per cell is size-independent at this size (memory-bound, "
                                f"working set >> last-level cache)")
         rconfig["step"] = (f"2 RK stages (computeA<KernelAdvectDiffuse> + update) + pressure_rhs + pressure_rhs1 + {K} BiCGSTAB "
-                           f"iterations + pressure correction, each operator timed separately (median of >= 5 reps) and composed")
+                           f"iterations + pressure correction, each operator timed separately (median of {args.steps} reps) and composed")
         line = {"impl": "reference", "metric": "Mcell-updates/s (advect+diffuse+Poisson iter)", "value": cb["value"],
                 "unit": "Mcell-updates/s", "n_gpus": 0, "steps": args.steps, "warmup": args.warmup,
                 "ms_per_step": cb["ms_per_step"], "higher_is_better": True, "scaling": "strong",
@@ -390,6 +434,11 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     launches = sim.launch_count() - l0
     dt_last, it_last, err_last = sim.step_result()
+    if args.dump_outputs:
+        _l.check(lib.cup2d_field_download(H, 0, vel_out.data_ptr()))
+        _l.check(lib.cup2d_field_download(H, 4, pres_out.data_ptr()))
+        dump_outputs(args.dump_outputs, np, dist, rank, order, sim.nbx, vel_out.numpy(), pres_out.numpy(),
+                     (dt_last, it_last, err_last))
     ms_per_step = ms / args.steps
     value = cells * (2 + K) / (ms_per_step * 1e-3) / 1e6
 
@@ -443,7 +492,7 @@ def main():
     if e2e is not None and world == 1 and not args.no_pipeline:
         try:
             outs = [(torch.empty_like(vel_h).pin_memory(), torch.empty_like(pres_h).pin_memory()) for _ in range(2)]
-            njobs = max(args.steps, 12)
+            njobs = args.steps
 
             def batch(n):
                 return sim.pipelined_steps(((vel_h.data_ptr(), pres_h.data_ptr(), outs[j % 2][0].data_ptr(), outs[j % 2][1].data_ptr())

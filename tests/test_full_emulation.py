@@ -427,24 +427,40 @@ def test_measurement_variants_keep_parity():
     assert r.returncode == 0 and " passed" in r.stdout, r.stdout[-1500:]
 
 
+def _emulated_driver(name, emulated_library, tmp_path):
+    """oracle/_ref/<name>.o (the reference's loop with the drop-in fragments spliced in, compiled by build()) linked against the
+    emulated library.  Only the link step runs here, so the reference's sources are not needed, only what build() left in
+    oracle/_ref/; skipped where that was not built."""
+    objs = [os.path.join(ROOT, "oracle", "_ref", f) for f in (name + ".o", "ref_spmat_cpu.o")]
+    if not all(os.path.exists(o) for o in objs):
+        pytest.skip(f"oracle/_ref/{name}.o not built")
+    emu_dir = os.path.dirname(emulated_library)
+    exe = str(tmp_path / (name + "_emu"))
+    subprocess.run(["g++", "-fopenmp", "-o", exe, *objs, f"-L{emu_dir}", "-lcup2d_emu", f"-Wl,-rpath,{emu_dir}"], check=True)
+    return exe
+
+
+def _reference_harness():
+    exe = os.path.join(ROOT, "oracle", "_ref", "ref_harness")
+    if not os.path.exists(exe):
+        pytest.skip("oracle/_ref/ref_harness not built")
+    return exe
+
+
 @pytest.mark.parametrize("name", ["steps_L2_random_k8", "steps_L3_tg_k15"])
 def test_reference_time_loop_on_the_emulated_library(emulated_library, golden_dir, name, tmp_path):
     """the drop-in boundary for the operators, end to end: the reference's OWN time loop (unmodified main.cpp with lines
     6607-6642 and 7007-7187 replaced at build time by dropin/patched_loop_*.inc + dropin/b200_loop_glue.h), linked against the
     emulated library, against the steps the unmodified reference produced (tests/golden/steps_*.npz)"""
     import numpy as np
-    if not os.path.exists("/root/reference/main.cpp"):
-        pytest.skip("needs the reference sources to build the patched driver (build container only)")
-    emu_dir = os.path.dirname(emulated_library)
-    subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "ref_patched", f"LIBDIR={emu_dir}", "LIBNAME=cup2d_emu",
-                    "PATCHED=ref_harness_patched_emu", f"RPATH={emu_dir}"], check=True, stdout=subprocess.DEVNULL)
+    exe = _emulated_driver("ref_harness_patched", emulated_library, tmp_path)
     g = np.load(os.path.join(golden_dir, name + ".npz"))
     L, K, ns = int(g["L"]), int(g["kiter"]), len(g["dt"])
     N = 8 << L
     z = np.zeros((N, N))
     fin, fout = tmp_path / "in.bin", tmp_path / "out.bin"
     np.concatenate([a.ravel() for a in (g["u0"], g["v0"], g["p0"], z, z, z)]).tofile(fin)
-    subprocess.run([os.path.join(ROOT, "oracle", "_ref", "ref_harness_patched_emu"), "steps", str(L), repr(float(g["nu"])),
+    subprocess.run([exe, "steps", str(L), repr(float(g["nu"])),
                     repr(float(g["cfl"])), str(ns), str(K), str(fin), str(fout)], check=True, stderr=subprocess.DEVNULL,
                    env=dict(os.environ, OMP_NUM_THREADS="1", CUP2D_B200_MAX_ITER=str(K)), timeout=900)
     raw = np.fromfile(fout).reshape(ns, 1 + 5 * N * N)
@@ -460,17 +476,13 @@ def test_reference_loop_with_bodies_device_resident_on_the_emulated_library(emul
     6945-6979, 6981-7187) while ongrid(), the 3x3 rigid-motion solve, the collision model and the forces stay on the host —
     two interacting fish, 4 steps (the last one with a collision), against the unmodified reference run the same way"""
     import numpy as np
-    if not os.path.exists("/root/reference/main.cpp"):
-        pytest.skip("needs the reference sources to build the patched driver (build container only)")
-    emu_dir = os.path.dirname(emulated_library)
-    subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "ref", "ref_resident", f"LIBDIR={emu_dir}", "LIBNAME=cup2d_emu",
-                    "RESIDENT=ref_harness_resident_emu", f"RPATH={emu_dir}"], check=True, stdout=subprocess.DEVNULL)
+    exes = (_reference_harness(), _emulated_driver("ref_harness_resident", emulated_library, tmp_path))
     env = dict(os.environ, OMP_NUM_THREADS="1", CUP2D_B200_MAX_ITER="5",
                CUP2D_REF_SHAPES="angle=0 L=0.8 xpos=0.52 ypos=0.44\n angle=175 L=0.8 xpos=0.47 ypos=0.56")
     outs = []
-    for exe in ("ref_harness", "ref_harness_resident_emu"):
-        out = tmp_path / (exe + ".bin")
-        subprocess.run([os.path.join(ROOT, "oracle", "_ref", exe), "fsteps", "4", "4", "5", str(out)], check=True,
+    for exe in exes:
+        out = tmp_path / (os.path.basename(exe) + ".bin")
+        subprocess.run([exe, "fsteps", "4", "4", "5", str(out)], check=True,
                        stderr=subprocess.DEVNULL, stdout=subprocess.DEVNULL, env=env, timeout=900)
         outs.append(np.fromfile(out))
     N = 128
@@ -507,18 +519,14 @@ def test_reference_amr_case_on_the_multi_level_path_emulated(emulated_library, t
     (By hand, both forms: 13 steps across a regrid 278 -> 281 blocks stay within 3e-15 / 1.3e-14 relative in velocity /
     pressure.)"""
     import numpy as np
-    if not os.path.exists("/root/reference/main.cpp"):
-        pytest.skip("needs the reference sources to build the patched driver (build container only)")
-    emu_dir = os.path.dirname(emulated_library)
-    subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "ref", f"ref_{form}", f"LIBDIR={emu_dir}", "LIBNAME=cup2d_emu",
-                    f"{form.upper()}=ref_harness_{form}_emu", f"RPATH={emu_dir}"], check=True, stdout=subprocess.DEVNULL)
+    exes = (_reference_harness(), _emulated_driver(f"ref_harness_{form}", emulated_library, tmp_path))
     # amrresident also takes adapt()'s tagging field from the device (cup2d_amr_adapt_tags, eleven adapt() calls in this
     # short run, the initial refinement included): the mesh must be the reference's from the start
     env = dict(os.environ, OMP_NUM_THREADS="1", CUP2D_B200_MAX_ITER="5", CUP2D_B200_AMR_FAST="1", CUP2D_B200_AMR_TAGS="1")
     runs = []
-    for exe in ("ref_harness", f"ref_harness_{form}_emu"):
-        out = tmp_path / (exe + ".bin")
-        subprocess.run([os.path.join(ROOT, "oracle", "_ref", exe), "asteps", "8", str(steps), "5", str(out)], check=True,
+    for exe in exes:
+        out = tmp_path / (os.path.basename(exe) + ".bin")
+        subprocess.run([exe, "asteps", "8", str(steps), "5", str(out)], check=True,
                        stderr=subprocess.DEVNULL, stdout=subprocess.DEVNULL, env=env, timeout=1500)
         runs.append(_parse_asteps(out))
     assert len(runs[0]) == len(runs[1]) == steps
